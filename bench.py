@@ -58,6 +58,23 @@ WORKLOADS = {
                           name="seedx_comprehension_448 (BASELINE.json configs[1])", metric="comprehension text tokens/sec"),
 }
 PROMPT_LEN = {2: 182, 5: 380}          # <s> [INST] + views x 66 span tokens + 32 text tokens + [/INST]\n + <img> (SeedXEngine.build_prompt, SynthTokenizer)
+DUMP_BYTES = 64 * 10 ** 6               # --dump-outputs: bytes written in all, .npy headers included
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as out_dir/<name>.npy in float32 (uint8 pixels and token ids are exact in it).  When the arrays exceed
+    DUMP_BYTES together, each is replaced by a sample of its flattened elements, in index order, drawn with a fixed seed and sized in
+    proportion to the array: runs with the same arguments write the same elements, so two builds compare output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in arrays.items()}
+    budget = (DUMP_BYTES - 1024 * len(arrays)) // 4
+    total = sum(a.size for a in arrays.values())
+    for name, a in arrays.items():
+        if total > budget:
+            idx = np.random.default_rng(0).choice(a.size, a.size * budget // total, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def unit_counts(workload, steps=50):
@@ -366,13 +383,15 @@ def run_comprehension(args, eng, rank, world, peaks_, cpu_base):
         e1.record()
         torch.cuda.synchronize()
         assert len(out["ids"]) == new_tok
-        return sdist.max_over_ranks(e0.elapsed_time(e1), "cuda"), _lib.launch_count() - n0
+        return sdist.max_over_ranks(e0.elapsed_time(e1), "cuda"), _lib.launch_count() - n0, out
 
     for _ in range(args.warmup):
         step(False)
     with ClockSampler(int(os.environ.get("LOCAL_RANK", "0"))) as cs:
-        ms_dev, launches = timed(False)
-        ms_e2e, _ = timed(True)
+        ms_dev, launches, last = timed(False)
+        ms_e2e, _, _ = timed(True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"text_ids": last["ids"]})
     trace.enable(True)
     trace.mark("start")
     step(False)
@@ -412,7 +431,14 @@ def main():
     ap.add_argument("--small", action="store_true", help="debug: tiny models (NOT a valid benchmark)")
     ap.add_argument("--workload", default="i2i", choices=sorted(WORKLOADS),
                     help="i2i (default, the headline metric) | edit (configs[3]) | anyres (configs[4]) | comprehension (configs[1], tokens/s)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step of the headline window returned (rank 0: images, text token ids) "
+                         "as DIR/<name>.npy, float32, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours; the reference arm times single stage units")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -427,6 +453,7 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: there is no CPU fallback for the product path")
     torch.cuda.set_device(local)
+    torch.manual_seed(0)            # the denoise loop draws its latent noise from the default generators: same arguments, same inputs
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
@@ -521,27 +548,34 @@ def main():
             log(f"warmup {i}: {eng.stage_ms()}")
     sync()
 
-    def timed(e2e):
+    def timed(e2e, keep=False):
         sync()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         n0 = _lib.launch_count()
         stages = []
         e0.record()
         for _ in range(args.steps):
-            step(e2e)
+            u8 = step(e2e)
             stages.append(eng._events)
         e1.record()
         sync()
+        if keep:                                       # outside the timed window, before the next step can reuse the buffers
+            kept["images"] = u8.cpu().numpy()
+            if W["text_tokens"]:
+                kept["text_ids"] = eng.last_text_ids
         ms = sdist.max_over_ranks(e0.elapsed_time(e1), "cuda")
         st = {k: statistics.mean(a.elapsed_time(b) for (a, b) in [(ev[i], ev[i + 1]) for ev in stages])
               for i, k in enumerate(("vit_ms", "llm_ms", "detok_ms"))}
         return ms, _lib.launch_count() - n0, st
 
+    kept = {}
     if rank == 0:       # one nvidia-smi poller per job (8 of them would only add host noise); rank 0's GPU stands for the box
         with ClockSampler(local) as cs:
-            ms_dev, launches, stages = timed(e2e=False)
+            ms_dev, launches, stages = timed(e2e=False, keep=bool(args.dump_outputs))
             ms_e2e, _, _ = timed(e2e=True)
         clocks = cs.summary()
+        if kept:
+            dump_outputs(args.dump_outputs, kept)
     else:
         ms_dev, launches, stages = timed(e2e=False)
         ms_e2e, _, _ = timed(e2e=True)

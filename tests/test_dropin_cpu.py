@@ -1,9 +1,9 @@
 """Drop-in surface checked without a GPU: prompt layouts, grounding post-processing, the launcher for unmodified reference scripts, and
-(in the build container, where /root/reference exists) a static check that every keyword the reference's entry scripts pass to the
-factories / generate() / init_pipe() is a named parameter of the replacement."""
+checks against the reference's own entry scripts, configs, goldens and pre-processing.  What those checks compare against was recorded
+from the reference tree into tests/golden/reference_surface.json (tests/golden/make_reference_surface.py), so they run without it."""
 import ast
-import glob
 import inspect
+import json
 import os
 import subprocess
 import sys
@@ -14,8 +14,11 @@ import torch
 from seedx_b200 import synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+sys.path.insert(0, GOLDEN)
+import make_reference_surface as surface  # noqa: E402
+
+REF = json.load(open(os.path.join(GOLDEN, "reference_surface.json")))
 
 
 def test_chat_prompt_layout_single_and_multi_turn():
@@ -44,16 +47,6 @@ def test_chat_prompt_layout_single_and_multi_turn():
         demo.chat_prompt(tok, ["q1", "a1"])
 
 
-def _ref_function(path, name):
-    """source of one top-level function of a reference script, executed in an empty namespace (no reference code is stored here)"""
-    tree = ast.parse(open(path).read())
-    fn = next(n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == name)
-    ns = {}
-    import re
-    exec(compile(ast.Module(body=[fn], type_ignores=[]), path, "exec"), {"re": re}, ns)
-    return ns[name]
-
-
 def test_extract_box_and_pixel_corners():
     from seedx_b200 import demo
     s = "The mask <box_start><loc-112><loc-56><loc-40><loc-20><box_end> and <box_start><loc-0><loc-223><loc-10><loc-5><box_end>."
@@ -62,10 +55,10 @@ def test_extract_box_and_pixel_corners():
     # (x_center, y_center, w, h) in 224 bins on a 448 x 896 image
     assert demo.box_to_pixels([112, 56, 40, 20], 448, 896) == (184, 184, 264, 264)
     assert demo.box_to_pixels([0, 223, 10, 5], 448, 896) == (-10, 882, 10, 902)
-    if os.path.isdir(REF):
-        ref = _ref_function(os.path.join(REF, "src/inference/eval_img2text_seed_x_i.py"), "extract_box")
-        for t in (s, "none", "<box_start><loc-7><box_end><box_start><box_end>", "<box_start>a<loc-1>b<loc-22>c<box_end>"):
-            assert demo.extract_box(t) == ref(t)
+    # the reference's own extract_box (eval_img2text_seed_x_i.py) on the same strings
+    assert [t for t, _ in REF["extract_box"]] == [s, "none", "<box_start><loc-7><box_end><box_start><box_end>", "<box_start>a<loc-1>b<loc-22>c<box_end>"]
+    for t, want in REF["extract_box"]:
+        assert demo.extract_box(t) == want, t
 
 
 def test_visualize_bbox_draws_the_rectangle(tmp_path):
@@ -104,87 +97,87 @@ def test_launcher_runs_a_reference_style_script(tmp_path):
     assert r.stdout.strip().endswith("OK True sibling import ok proj 32 32330"), r.stdout
 
 
-# ---- static call-surface check against the reference's own entry scripts ---------------------------------------------------------------
-def _calls(tree):
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Call) and isinstance(node.func, ast.Attribute):
-            yield node
-
-
+# ---- checks against the reference's own entry scripts, configs, goldens and pre-processing (recorded in tests/golden/reference_surface.json) --
 def _named_params(fn):
     return {p.name for p in inspect.signature(fn).parameters.values() if p.kind in (p.POSITIONAL_OR_KEYWORD, p.KEYWORD_ONLY)}
 
 
-@needs_ref
 def test_reference_scripts_only_use_keywords_the_replacement_names():
     from seedx_b200 import compat
     compat.install()
     from seedx_b200.adapter import SDXLAdapter, SDXLAdapterWithLatentImage
     from seedx_b200.agent import ContinuousLVLM
     from seedx_b200.sdxl import AutoencoderKL, EulerDiscreteScheduler, UNet2DConditionModel
-    scripts = sorted(glob.glob(os.path.join(REF, "src/inference/eval_*.py")))
+    scripts = REF["entry_scripts"]
     assert len(scripts) == 7
     seen = 0
-    for path in scripts:
-        tree = ast.parse(open(path).read())
-        src = open(path).read()
-        edit = "with_latent_image" in src
-        adapter_cls = SDXLAdapterWithLatentImage if edit else SDXLAdapter
-        for c in _calls(tree):
-            kws = {k.arg for k in c.keywords if k.arg is not None}
-            owner = c.func.value.id if isinstance(c.func.value, ast.Name) else None
-            if c.func.attr == "generate" and owner == "agent_model":
+    for name, script in sorted(scripts.items()):
+        adapter_cls = SDXLAdapterWithLatentImage if script["edit"] else SDXLAdapter
+        for c in script["calls"]:
+            kws, owner = set(c["keywords"]), c["owner"]
+            if c["attr"] == "generate" and owner == "agent_model":
                 target = ContinuousLVLM.generate
-            elif c.func.attr == "generate" and owner == "adapter":
+            elif c["attr"] == "generate" and owner == "adapter":
                 target = adapter_cls.generate
-            elif c.func.attr == "init_pipe" and owner == "adapter":
+            elif c["attr"] == "init_pipe" and owner == "adapter":
                 target = adapter_cls.init_pipe
-            elif c.func.attr == "from_pretrained" and owner in ("AutoencoderKL", "UNet2DConditionModel", "EulerDiscreteScheduler"):
+            elif c["attr"] == "from_pretrained" and owner in ("AutoencoderKL", "UNet2DConditionModel", "EulerDiscreteScheduler"):
                 target = {"AutoencoderKL": AutoencoderKL, "UNet2DConditionModel": UNet2DConditionModel,
                           "EulerDiscreteScheduler": EulerDiscreteScheduler}[owner].from_pretrained
             else:
                 continue
             missing = kws - _named_params(target)
-            assert not missing, f"{os.path.basename(path)}:{c.lineno} passes {sorted(missing)} which {target.__qualname__} does not name"
+            assert not missing, f"{name}:{c['line']} passes {sorted(missing)} which {target.__qualname__} does not name"
             seen += 1
     assert seen >= 20, seen
 
 
-@needs_ref
+def _import_block_module(block):
+    """the recorded import block of one entry script as a module: its imports and its `setup_root(...)` statement, in order"""
+    body = []
+    for st in block:
+        if "import" in st:
+            body.append(ast.Import(names=[ast.alias(name=n, asname=a) for n, a in st["import"]]))
+        elif "from" in st:
+            body.append(ast.ImportFrom(module=st["from"], names=[ast.alias(name=n, asname=a) for n, a in st["names"]], level=st["level"]))
+        else:
+            c = st["call"]
+            args = [ast.Name(id=a["name"], ctx=ast.Load()) if isinstance(a, dict) else ast.Constant(a) for a in c["args"]]
+            func = ast.Attribute(value=ast.Name(id=c["owner"], ctx=ast.Load()), attr=c["attr"], ctx=ast.Load())
+            body.append(ast.Expr(ast.Call(func=func, args=args, keywords=[ast.keyword(arg=k, value=ast.Constant(v)) for k, v in c["kwargs"].items()])))
+    return ast.fix_missing_locations(ast.Module(body=body, type_ignores=[]))
+
+
 def test_import_block_of_every_reference_entry_script_executes_under_the_stand_ins():
     """the statements every reference entry script runs before touching a model — its top-level imports (incl. `from diffusers import …,
     Transformer2DModel` and the sibling `from any_res import …`) and `pyrootutils.setup_root` — execute against this repo exactly as
     `python -m seedx_b200.run <script>` would run them (compat.install() + script directory on sys.path); a missing name fails here, not on a GPU box"""
-    scripts = sorted(glob.glob(os.path.join(REF, "src/inference/eval_*.py")))
+    scripts = REF["entry_scripts"]
     assert len(scripts) == 7
+    blocks = {name: ast.unparse(_import_block_module(s["import_block"])) for name, s in sorted(scripts.items())}
+    for name, s in scripts.items():
+        assert len(s["import_block"]) >= 7, name
+        assert s["import_block"][-1]["call"]["attr"] == "setup_root", name
     code = r'''
-import ast, os, sys
+import os, sys
 sys.path.insert(0, %r)
 from seedx_b200 import compat
 compat.install()
 sys.path.insert(0, os.path.join(%r, "src", "inference"))      # what seedx_b200.run does for the sibling import
-for path in %r:
-    tree = ast.parse(open(path).read())
-    block = []
-    for node in tree.body:
-        is_setup = isinstance(node, ast.Expr) and isinstance(node.value, ast.Call) and getattr(node.value.func, "attr", "") == "setup_root"
-        if isinstance(node, (ast.Import, ast.ImportFrom)) or is_setup:
-            block.append(node)
-    assert len(block) >= 7, path
+for name, block in %r.items():
     # __file__ of the script as the launcher sees it: the same relative location inside THIS repo
-    ns = {"__name__": "not_main", "__file__": os.path.join(%r, "src", "inference", os.path.basename(path))}
-    exec(compile(ast.Module(body=block, type_ignores=[]), path, "exec"), ns)
+    ns = {"__name__": "not_main", "__file__": os.path.join(%r, "src", "inference", name)}
+    exec(compile(block, name, "exec"), ns)
     import diffusers
     for n in ("AutoencoderKL", "UNet2DConditionModel", "EulerDiscreteScheduler"):
         assert ns[n] is getattr(diffusers, n)
-    print("ok", os.path.basename(path))
-''' % (ROOT, ROOT, scripts, ROOT)
+    print("ok", name)
+''' % (ROOT, ROOT, blocks, ROOT)
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-3000:]
     assert r.stdout.count("ok eval_") == 7, r.stdout
 
 
-@needs_ref
 def test_reference_yaml_targets_resolve_with_identical_keys():
     """every inference YAML of the reference has a twin here with the same `_target_`s and keys (values may differ only in comments)"""
     import yaml
@@ -194,6 +187,7 @@ def test_reference_yaml_targets_resolve_with_identical_keys():
              "clm_models/llm_seed_x_edit.yaml", "clm_models/llm_seed_x_lora.yaml", "clm_models/agent_seed_x.yaml", "clm_models/agent_seed_x_i.yaml",
              "clm_models/agent_seed_x_edit.yaml", "sdxl_adapter/sdxl_qwen_vit_resampler_l4_q64_pretrain_no_normalize.yaml",
              "sdxl_adapter/sdxl_qwen_vit_resampler_l4_q64_full_with_latent_image_pretrain_no_normalize.yaml"]
+    assert sorted(REF["configs"]) == sorted(names)
 
     def targets(o, acc):
         if isinstance(o, dict):
@@ -205,7 +199,7 @@ def test_reference_yaml_targets_resolve_with_identical_keys():
 
     for n in names:
         ours = yaml.safe_load(open(os.path.join(ROOT, "configs", n)))
-        ref = yaml.safe_load(open(os.path.join(REF, "configs", n)))
+        ref = REF["configs"][n]
         assert ours == ref, n
         for t in targets(ours, []):
             if t.startswith(("src.", "peft.")):
@@ -213,63 +207,33 @@ def test_reference_yaml_targets_resolve_with_identical_keys():
                 assert callable(compat._locate(t)), t
 
 
-@needs_ref
-def test_goldens_regenerate_bit_identically_from_the_reference(tmp_path):
-    """tests/golden/*.pt ARE the outputs of the reference's own modules: running the generator again (imports /root/reference, binds `src` to it
-    explicitly) reproduces every committed tensor exactly"""
-    env = dict(os.environ, SEEDX_GOLDEN_OUT=str(tmp_path))
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "golden", "make_golden.py")], cwd=ROOT, env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stderr[-3000:]
-
-    def same(a, b, path):
-        if torch.is_tensor(a):
-            assert torch.is_tensor(b) and a.shape == b.shape and torch.equal(a, b), path
-        elif isinstance(a, dict):
-            assert a.keys() == b.keys(), path
-            for k in a:
-                same(a[k], b[k], f"{path}/{k}")
-        elif isinstance(a, (list, tuple)):
-            assert len(a) == len(b), path
-            for i, (x, y) in enumerate(zip(a, b)):
-                same(x, y, f"{path}[{i}]")
-        else:
-            assert a == b, path
-
-    names = sorted(f for f in os.listdir(os.path.join(ROOT, "tests", "golden")) if f.endswith(".pt"))
-    assert names == sorted(f for f in os.listdir(tmp_path) if f.endswith(".pt")) and len(names) == 8
+def test_goldens_regenerate_bit_identically_from_the_reference():
+    """tests/golden/*.pt ARE the outputs of the reference's own modules: every committed tensor is bit-identical (dtype, shape, SHA-256 of
+    its bytes) and every other value equal to what tests/golden/make_golden.py wrote when it was run against the reference modules"""
+    names = sorted(f for f in os.listdir(GOLDEN) if f.endswith(".pt"))
+    assert names == sorted(REF["goldens"]) and len(names) == 8
     for f in names:
-        same(torch.load(os.path.join(ROOT, "tests", "golden", f)), torch.load(tmp_path / f), f)
+        got, want = surface.nested_digests(torch.load(os.path.join(GOLDEN, f))), REF["goldens"][f]
+        assert got.keys() == want.keys(), f
+        for k in want:
+            assert got[k] == want[k], f"{f}{k}"
 
 
-@needs_ref
 def test_anyres_preprocessing_equals_the_reference_on_random_sizes():
-    """seedx_b200.preprocess vs the reference's own functions (imported in a subprocess so its `src` package cannot shadow this repo's shims):
-    grid choice, tile order, patch positions and pixel values, bit for bit, on 60 random image sizes and both transform modes"""
-    code = r'''
-import sys, numpy as np, torch
-from PIL import Image
-sys.path.insert(0, "%s"); sys.path.insert(0, "%s/tests/golden")
-from _ref_import import ref_module
-ar, tr = ref_module("src.inference.any_res"), ref_module("src.processer.transforms")
-from seedx_b200 import preprocess as pp
-base = 448
-grids = [[base * int(g[0]), base * int(g[2])] for g in ["1x1", "1x2", "1x3", "2x1", "3x1", "1x4", "4x1", "2x2"]]
-rng = np.random.RandomState(7)
-n = 0
-for i in range(60):
-    w, h = int(rng.randint(40, 2600)), int(rng.randint(40, 2600))
-    img = Image.fromarray(rng.randint(0, 255, (h, w, 3), dtype=np.uint8))
-    use = grids if i %% 3 else grids[:1]
-    v0, p0 = ar.process_anyres_image(img, tr.get_transform("clip", keep_ratio=False, image_size=base), use, base)
-    v1, p1 = pp.process_anyres_image(img, pp.get_transform("clip", keep_ratio=False, image_size=base), use, base)
-    assert v0.shape == v1.shape and torch.equal(p0, p1) and torch.equal(v0, v1), (w, h)
-    if i %% 10 == 0:
-        k0 = tr.get_transform("clip", keep_ratio=True, image_size=base)(img)
-        k1 = pp.get_transform("clip", keep_ratio=True, image_size=base)(img)
-        assert torch.equal(k0, k1), (w, h)
-    n += 1
-print("checked", n)
-''' % (ROOT, ROOT)
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=900, cwd=ROOT)
-    assert r.returncode == 0, r.stderr[-3000:]
-    assert r.stdout.strip().endswith("checked 60")
+    """seedx_b200.preprocess vs the reference's own functions: grid choice, tile order, patch positions and pixel values, bit for bit
+    (dtype, shape and SHA-256 of the reference's outputs), on 60 random image sizes and both transform modes"""
+    from seedx_b200 import preprocess as pp
+    base = surface.ANYRES_BASE
+    cases = REF["anyres"]
+    assert len(cases) == 60
+    n = 0
+    for (i, w, h, img, grids, keep), want in zip(surface.anyres_cases(), cases):
+        assert (i, w, h) == (want["i"], want["w"], want["h"])
+        v1, p1 = pp.process_anyres_image(img, pp.get_transform("clip", keep_ratio=False, image_size=base), grids, base)
+        assert surface.tensor_digest(v1) == want["views"] and surface.tensor_digest(p1) == want["patch_positions"], (w, h)
+        assert keep == ("keep_ratio" in want)
+        if keep:
+            k1 = pp.get_transform("clip", keep_ratio=True, image_size=base)(img)
+            assert surface.tensor_digest(k1) == want["keep_ratio"], (w, h)
+        n += 1
+    assert n == 60

@@ -96,6 +96,26 @@ def test_reference_arm_prints_the_contract_line():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0 and math.isfinite(line["value"])
 
 
+def test_bench_output_dump_is_float32_exact_and_sampled_reproducibly_over_budget(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: uint8 pixels and token ids land exactly in float32; over the byte budget every array is cut to the same
+    seeded sample of its elements on every run, in index order, and the files stay within the budget"""
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(5)
+    img = rng.integers(0, 256, (2, 64, 64, 3), dtype=np.uint8)
+    ids = [[7, 31000, 2], [5, 6, 32329]]
+    bench.dump_outputs(str(tmp_path / "a"), {"images": img, "text_ids": ids})
+    a_img, a_ids = np.load(tmp_path / "a" / "images.npy"), np.load(tmp_path / "a" / "text_ids.npy")
+    assert a_img.dtype == np.float32 and np.array_equal(a_img, img) and np.array_equal(a_ids, np.array(ids))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 20000)
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), {"images": img, "text_ids": ids})
+    b_img, c_img = np.load(tmp_path / "b" / "images.npy"), np.load(tmp_path / "c" / "images.npy")
+    assert b_img.ndim == 1 and 0 < b_img.size < img.size and np.array_equal(b_img, c_img)
+    assert sum(os.path.getsize(tmp_path / "b" / f) for f in os.listdir(tmp_path / "b")) <= 20000
+    assert np.isin(b_img, img.reshape(-1)).all()
+
+
 def test_reference_arm_under_torchrun_prints_once():
     """launched the way the driver launches N>1 (torch.distributed.run, one process per rank): rank 0 alone times and prints the line,
     the other ranks exit 0 without output"""
